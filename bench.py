@@ -5,6 +5,7 @@
   python bench.py --impl reference --steps K --warmup W    # the reference's CPU worker-pool path (oracle port) on the host cores
   torchrun --nproc-per-node N bench.py --gpus N ...        # N GPUs: key space sharded by the replicated-hash ring
   python bench.py --workload global ...                    # BASELINE config 5: GLOBAL hot keys + sync ticks (any N)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's responses as DIR/<field>.npy
 
 A "step" is one 65 536-request batch per GPU through the whole hot path (group -> probe -> bucket update -> response):
 ONE launch of the persistent batch kernel k_batch.  Workload at N = 1: BASELINE config 3 — 100 M resident keys, Zipf s = 1.1,
@@ -68,7 +69,13 @@ def parse_args():
     ap.add_argument("--traffic-probe", action="store_true", help=argparse.SUPPRESS)  # the ncu sub-process runs this
     ap.add_argument("--ncu-window", type=int, default=0,
                     help="profile this many extra steps between cudaProfilerStart/Stop (run under `ncu --profile-from-start off`)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the responses of the last timed step as DIR/<field>.npy (float64; with N > 1 "
+                         "every rank writes DIR/<field>_rank<r>.npy).  The inputs depend on the arguments alone; with --workload global "
+                         "the tick period is calibrated from wall-clock time, so the table state there depends on it too")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if not a.keys:
         a.keys = 10_000_000 if a.workload == "global" else 100_000_000
     return a
@@ -162,6 +169,13 @@ def gen_batch(rng, n, n_keys, created_at, zipf_s, dtype, global_hot=0, hits_mix=
     return reqs, ids
 
 
+def dump_outputs(out_dir, resp, suffix=""):
+    """The response records of one step as one float64 array per field (every value is an integer below 2^53: exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for f in resp.dtype.names:
+        np.save(os.path.join(out_dir, f"{f}{suffix}.npy"), resp[f].astype(np.float64))
+
+
 def batch_stats(ids):
     _, counts = np.unique(ids, return_counts=True)
     return dict(distinct=int(len(counts)), singles=int((counts == 1).sum()), repeated_keys=int((counts > 1).sum()),
@@ -187,7 +201,7 @@ def cpu_keys_that_fit(want):
     return int(max(1_000_000, min(want, (avail // 2) // 250)))
 
 
-def cpu_leg(n_keys, zipf_s, seconds, seed, steps=None, warmup=0, step_size=BATCH, min_seconds=2.0, from_keys=True):
+def cpu_leg(n_keys, zipf_s, seconds, seed, steps=None, warmup=0, step_size=BATCH, from_keys=True):
     """The oracle's worker-pool port (W = cores shard threads) over the same synthetic traffic.  from_keys: every step starts
     from the key strings (XXH64 + FNV-1 inside the timed call), like the reference's own path (client.go:39, workers.go:153)."""
     import oracle_py as O
@@ -207,13 +221,15 @@ def cpu_leg(n_keys, zipf_s, seconds, seed, steps=None, warmup=0, step_size=BATCH
         blob, offs = key_blob(ids)
         batches.append((reqs, blob, offs))
 
+    last = [None]
+
     def one(b):
         reqs, blob, offs = batches[b % len(batches)]
         pool.set_now(T0 + 1 + b)
         if from_keys:
-            pool.submit_keys(blob, offs, reqs, threads=cores)
+            last[0] = pool.submit_keys(blob, offs, reqs, threads=cores)
         else:
-            pool.submit_hashed(reqs, threads=cores)
+            last[0] = pool.submit_hashed(reqs, threads=cores)
         return pool.last_mt_seconds
     for w in range(max(warmup, 1)):
         one(w)
@@ -222,12 +238,13 @@ def cpu_leg(n_keys, zipf_s, seconds, seed, steps=None, warmup=0, step_size=BATCH
         if steps is None:
             if t_used >= seconds:
                 break
-        elif b >= steps and t_used >= min_seconds:
+        elif b >= steps:
             break
         t_used += one(b)
         done += step_size
         b += 1
-    return dict(value=done / t_used, seconds=t_used, steps=b, cores=cores, fill_seconds=t_fill, keys=n_keys, step_size=step_size)
+    return dict(value=done / t_used, seconds=t_used, steps=b, cores=cores, fill_seconds=t_fill, keys=n_keys, step_size=step_size,
+                last_responses=last[0])
 
 
 def run_reference(args):
@@ -235,10 +252,11 @@ def run_reference(args):
     if rank != 0:
         return
     keys = args.cpu_keys or cpu_keys_that_fit(args.keys)
-    # at least 2 s of timed CPU work whatever --steps says (a 20-step sample is 50 ms of cache-warm work); beyond 20 000 steps the
-    # batch is shrunk so that the whole run stays within about a minute
+    # exactly --steps timed steps; beyond 20 000 steps the batch is shrunk so that the whole run stays within about a minute
     step_size = BATCH if args.steps <= 20000 else max(2048, int(BATCH * 20000 / args.steps) // 256 * 256)
-    r = cpu_leg(keys, args.zipf, args.cpu_seconds, 0xB200 + 3, steps=args.steps, warmup=min(args.warmup, 20), step_size=step_size, min_seconds=2.0)
+    r = cpu_leg(keys, args.zipf, args.cpu_seconds, 0xB200 + 3, steps=args.steps, warmup=min(args.warmup, 20), step_size=step_size)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["last_responses"])
     sample = (f"{r['steps']} x {step_size}-request Zipf({args.zipf}) batches over {r['keys']:,} resident keys"
               + ("" if r["keys"] == args.keys else f" (the GPU arm holds {args.keys:,}: host memory bounds the CPU table)")
               + f", TOKEN/LEAKY 50/50, from key strings (XXH64 + FNV-1 inside the timed call), {r['cores']} worker threads, {r['seconds']:.1f} s timed")
@@ -493,6 +511,9 @@ def run_b200(args):
     barrier()
     progress("timed steps done")
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:  # before the legs below reuse the output buffers
+        last = d_outs[(args.warmup + args.steps - 1) % pool_n].cpu().numpy().view(g.RESP_DTYPE).reshape(BATCH)
+        dump_outputs(args.dump_outputs, last, f"_rank{rank}" if N > 1 else "")
     clocks_info = sampler.stop() if rank == 0 else None
     if dist is not None:
         tms = torch.tensor([ms], device=dev, dtype=torch.float64)

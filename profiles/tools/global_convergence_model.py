@@ -1,10 +1,11 @@
-import sys, importlib.util
-sys.path[:0] = ["/root/repo", "/root/repo/tests", "/root/repo/oracle"]
+import os, sys, importlib.util
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path[:0] = [ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "oracle")]
 import numpy as np
 import oracle_py as O
 from global_model import OracleCluster
 from workloads import bench_requests, T0
-spec = importlib.util.spec_from_file_location("bench_mod", "/root/repo/bench.py"); bench = importlib.util.module_from_spec(spec); spec.loader.exec_module(bench)
+spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py")); bench = importlib.util.module_from_spec(spec); spec.loader.exec_module(bench)
 W, n_keys, per_step, steps, pool_n = 2, 1000000, 16384, 2000, 32
 hot = n_keys // 100
 rng = [np.random.default_rng(100 + r) for r in range(W)]

@@ -4,6 +4,7 @@ CPU-only: runs in `pytest -m "not gpu"`.
 """
 import calendar
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
@@ -25,12 +26,21 @@ def test_xxh64_vectors():
 
 
 def test_xxh64_against_python_xxhash():
-    xxhash = pytest.importorskip("xxhash")
+    """python-xxhash's digests of these inputs are stored in tests/golden/xxh64_python_xxhash.npy (columns: seed 0, seed 12345),
+    so the comparison runs without the package; where it is installed the stored digests are checked against it too."""
+    try:
+        import xxhash
+    except ImportError:
+        xxhash = None
+    want = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "xxh64_python_xxhash.npy"))
     rng = np.random.default_rng(1)
-    for n in list(range(0, 70)) + [127, 128, 129, 1000]:
+    for j, n in enumerate(list(range(0, 70)) + [127, 128, 129, 1000]):
         b = rng.integers(0, 256, n, dtype=np.uint8).tobytes()
-        assert O.xxh64(b) == xxhash.xxh64(b, seed=0).intdigest()
-        assert O.xxh64(b, 12345) == xxhash.xxh64(b, seed=12345).intdigest()
+        assert O.xxh64(b) == int(want[j, 0])
+        assert O.xxh64(b, 12345) == int(want[j, 1])
+        if xxhash is not None:
+            assert int(want[j, 0]) == xxhash.xxh64(b, seed=0).intdigest()
+            assert int(want[j, 1]) == xxhash.xxh64(b, seed=12345).intdigest()
 
 
 def test_fnv_md5_vectors():
